@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: denoised frames/s at 512x512, 16-frame window, 20 DDIM steps (BASELINE.json, config 2).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
   (N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...)
 
 One "step" = one complete denoise of the workload: 20 DDIM steps of the Visual-Conditioned Parallel-Denoise loop
@@ -26,6 +26,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: no __pycache__ is written next to the sources
 
 DDIM_STEPS = 20
 WINDOW, OVERLAP = 16, 4
@@ -48,7 +49,15 @@ def parse():
     ap.add_argument("--controlnet", action="store_true", help="config-4 style: ControlNet encoder per window-step")
     ap.add_argument("--cpu-frames", type=int, default=4, help="frames of the bounded cpu_baseline sample (GPU arm)")
     ap.add_argument("--ref-frames", type=int, default=16, help="frames of one reference-arm step (16 = the config-2 window)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the denoised latents of the last timed step to DIR/latents.npy (float32); the inputs are "
+                         "seeded, so two builds run with the same arguments can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "musev_b200":
+        ap.error("--dump-outputs needs --impl musev_b200")
+    return args
 
 
 def video_frames(n_gpus: int) -> int:
@@ -379,6 +388,12 @@ def main():
                 "traffic": traffic, "traffic_unit": "bytes/launch", "traffic_source": traffic_src, "launches_per_step": gemm_n, "avg_launch_ms": gemm_ms / max(gemm_n, 1),
                 "algorithmic_tflop_per_forward": fl["gemm"] / 1e12,
                 "step_share": {k: round(v["ms"], 2) for k, v in prof.items()}}
+
+    if args.dump_outputs and rank == 0:
+        # `res` is what the last step of timed region 1 returned; the latents are replicated on every rank
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "latents.npy"), res.float().cpu().numpy())
 
     sys.stdout.flush()
     os.dup2(saved_stdout, 1)

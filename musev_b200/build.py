@@ -39,15 +39,17 @@ def _sources() -> list[str]:
 
 
 def _digest() -> str:
+    # names relative to the repository (not absolute paths), so that a checkout moved or copied elsewhere with its
+    # built library is not rebuilt
     h = hashlib.sha256()
-    files = sorted(os.listdir(CSRC)) + [os.path.join(INCLUDE, f) for f in sorted(os.listdir(INCLUDE))]
-    for f in files:
-        p = f if os.path.isabs(f) else os.path.join(CSRC, f)
+    repo = os.path.dirname(PKG_DIR)
+    files = [os.path.join(CSRC, f) for f in sorted(os.listdir(CSRC))] + [os.path.join(INCLUDE, f) for f in sorted(os.listdir(INCLUDE))]
+    for p in files:
         if os.path.isfile(p):
-            h.update(p.encode())
+            h.update(os.path.relpath(p, repo).encode())
             with open(p, "rb") as fh:
                 h.update(fh.read())
-    h.update(" ".join(NVCC_FLAGS).encode())
+    h.update(" ".join(f for f in NVCC_FLAGS if f != INCLUDE).encode())
     return h.hexdigest()
 
 
